@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — ray-samples/sec of the per-ray-sample hot path (march -> hash-grid -> fused MLPs -> composite) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one 1024x1024 frame of BASELINE config 3 (random-weight network_ff field, ball occupancy, bound 1, dt_gamma 0,
@@ -13,6 +13,8 @@ MLPs), measured live with CUDA events around every launch of one extra frame.  `
 random and ray-coherent samples through the fused field kernel and through the stand-alone grid encoder).
 `cpu_baseline` / `--impl reference`: the reference has no CPU implementation of this path (SURVEY F1), so the CPU arm is
 the oracle port (oracle/ntx_oracle.c, OpenMP over all host cores) rendering a strided sub-sample of the same frame.
+`--dump-outputs DIR` writes the frame the last timed step returned (image, depth, weights_sum) as DIR/<name>.npy in float32; the
+scene is seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -184,7 +186,10 @@ def main():
     ap.add_argument("--impl", default="ntx", choices=["ntx", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg2 / roofline side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step returned as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -235,11 +240,13 @@ def main():
             return res
         return render.gather_frame(out, N)
 
+    last = {}
+
     def step_device():
         # this rank's (resident) shard of the frame, rendered straight into its planar send block, + the exchange and the assembly
         # kernel (config 4); one GPU: the frame
         out = render.render_rays(field, my_o, my_d, bits, 1, 128, block_rows=n_max, cache_mip=True, block_out=exchange.block() if exchange is not None else None)
-        return finish(out)
+        last["out"] = finish(out)
 
     def barrier():
         if world > 1:
@@ -280,6 +287,13 @@ def main():
     launches = (L.launches - l0) // K
     clocks = sampler.stop() if rank == 0 else None
     value = samples_per_frame / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in last["out"].items():
+            if torch.is_tensor(t):
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
+    last.clear()
 
     # ---- end to end: rays from pinned host memory each step, image + depth read back each step --------------------
     h_o, h_d = my_o.cpu().pin_memory(), my_d.cpu().pin_memory()

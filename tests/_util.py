@@ -33,6 +33,118 @@ def ref(name):
     return mod
 
 
+# ------------------------------------------------------------------------------------------------ stored reference outputs
+REFERENCE_OUTPUTS = os.path.join(GOLDEN, "reference_outputs.npz")
+_RECORD_TO = os.environ.get("NTX_RECORD_REFERENCE")      # path: run the reference live (oracle/_ref) and store what it returned
+_stored = None
+_recorded = {}
+FULL_BYTES = 512             # arrays up to this size are stored whole; larger ones as a sample of elements plus a digest of the whole
+SAMPLE = 128                 # elements kept of an array compared to a tolerance (of one compared exactly: EXACT_SAMPLE, for the message)
+EXACT_SAMPLE = 16
+
+
+def _canonical(a):
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":      # value equality like assert_array_equal: -0 == +0, any NaN == any NaN
+        a = np.where(np.isnan(a), np.array(np.nan, a.dtype), a + a.dtype.type(0))
+    return a
+
+
+def _digest(a):
+    import hashlib
+    a = _canonical(a)
+    return np.frombuffer(hashlib.sha256(str((a.dtype.str, a.shape)).encode() + a.tobytes()).digest(), np.uint8)
+
+
+def _sample_index(key, size, n):
+    import zlib
+    return np.sort(np.random.default_rng(zlib.crc32(key.encode())).choice(size, min(n, size), replace=False))
+
+
+class Recorded:
+    """An output of the reference: whole (`index` is None) or the elements `index` of the flattened array, with its SHA-256 `digest`."""
+
+    def __init__(self, sample, index=None, digest=None, shape=None):
+        self.sample, self.index, self.digest, self.shape = sample, index, digest, shape
+
+    def take(self, a):
+        """the same elements of one of our arrays"""
+        a = np.asarray(a)
+        if self.shape is not None:
+            assert a.shape == tuple(self.shape), (a.shape, tuple(self.shape))
+        return a if self.index is None else a.reshape(-1)[self.index]
+
+    def assert_equal(self, a, msg=""):
+        """our array equals the reference's, element for element (the whole array, not only the stored sample)"""
+        np.testing.assert_array_equal(self.take(a), self.sample, err_msg=msg)
+        if self.digest is not None:
+            assert np.array_equal(_digest(a), self.digest), "%s: equal on the %d stored elements, different elsewhere" % (msg, len(self.index))
+
+
+def save_packed(path, arrays):
+    """many small arrays as one .npz of five (an .npz entry costs a few hundred bytes of zip headers)"""
+    keys = sorted(arrays)
+    vals = [np.asarray(arrays[k]) for k in keys]
+    np.savez_compressed(path, keys=np.array(keys), dtypes=np.array([v.dtype.str for v in vals]), ndims=np.array([v.ndim for v in vals], np.int64),
+                        dims=np.array([d for v in vals for d in v.shape], np.int64), blob=np.frombuffer(b"".join(v.tobytes() for v in vals), np.uint8))
+
+
+def load_packed(path):
+    z = np.load(path)
+    out, at, d = {}, 0, 0
+    dims = z["dims"]
+    for k, dt, nd in zip(z["keys"], z["dtypes"], z["ndims"]):
+        shape = tuple(int(x) for x in dims[d:d + nd])
+        n = int(np.prod(shape)) * np.dtype(dt).itemsize
+        out[str(k)] = np.frombuffer(z["blob"][at:at + n].tobytes(), dt).reshape(shape)
+        at, d = at + n, d + nd
+    return out
+
+
+def _record(key, v):
+    if not _recorded:
+        import atexit
+        atexit.register(lambda: save_packed(_RECORD_TO, _recorded))
+        if os.path.exists(_RECORD_TO):
+            _recorded.update(load_packed(_RECORD_TO))
+    _recorded[key] = v
+
+
+def reference_output(key, compute, exact=False):
+    """What the reference's own CUDA kernels (oracle/_ref) computed for `key` on the test's seeded inputs.
+
+    The reference is not part of this repository: its outputs are stored in tests/golden/reference_outputs.npz, written by running
+    the GPU tests with NTX_RECORD_REFERENCE=<that file> on a B200 where oracle/build_ref.py has built oracle/_ref.  Only then is
+    `compute` called.  A scalar comes back as a float, an array as a Recorded: whole when it is small, else a fixed sample of its
+    elements (chosen from `key`) and the digest of the whole array.  `exact`: the array is only ever compared for equality, so the
+    digest decides and a few elements suffice."""
+    global _stored
+    n = EXACT_SAMPLE if exact else SAMPLE
+    if _RECORD_TO:
+        v = compute()
+        if np.ndim(v) == 0:
+            _record(key, np.float64(v))
+            return float(v)
+        v = np.ascontiguousarray(v)
+        if v.nbytes <= FULL_BYTES:
+            _record(key, v)
+            return Recorded(v)
+        index = _sample_index(key, v.size, n)
+        rec = Recorded(v.reshape(-1)[index], index, _digest(v), v.shape)
+        _record(key + ":sample", rec.sample)
+        _record(key + ":digest", rec.digest)
+        _record(key + ":shape", np.array(v.shape, np.int64))
+        return rec
+    if _stored is None:
+        _stored = load_packed(REFERENCE_OUTPUTS)
+    if key in _stored:
+        v = _stored[key]
+        return float(v) if v.ndim == 0 else Recorded(v)
+    assert key + ":sample" in _stored, "no stored reference output %r in %s" % (key, REFERENCE_OUTPUTS)
+    shape = _stored[key + ":shape"]
+    return Recorded(_stored[key + ":sample"], _sample_index(key, int(np.prod(shape)), n), _stored[key + ":digest"], shape)
+
+
 def ntx():
     import nerf_texture_b200
     nerf_texture_b200.install()

@@ -1,11 +1,5 @@
-"""Density-grid maintenance (SURVEY 8 f2): ntx_update_density_grid / nerf_texture_b200.density.update_extra_state against
-  * the reference's OWN, unmodified NeRFRenderer.update_extra_state (baseline/_ref/callers/nerf/renderer.py:567) running on the
-    drop-in packages, with its jitter pinned (torch.rand_like patched) so that both sides see the same positions;
-  * the CPU oracle (positions as renderer.py:590-598 computes them -> oracle field -> EMA-max -> packbits) on a small grid."""
-import copy
-import os
-import sys
-
+"""Density-grid maintenance (SURVEY 8 f2): ntx_update_density_grid / nerf_texture_b200.density.update_extra_state against the CPU
+oracle (positions as renderer.py:590-598 computes them -> oracle field -> EMA-max -> packbits) on a small grid."""
 import numpy as np
 import pytest
 import torch
@@ -13,59 +7,7 @@ import torch
 from _util import ntx, oracle
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = torch.device("cuda", 0) if torch.cuda.is_available() else None
-STAGED = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "callers", "nerf", "renderer.py"))
-
-
-def _random_model(bound=1):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    import run_reference_files as R
-    Net, _ = R.import_reference_network("ntx")       # the reference's nerf/network_ff.py on the compat packages
-    model = Net(encoding="hashgrid", bound=bound, cuda_ray=True)
-    g = torch.Generator().manual_seed(3)
-    with torch.no_grad():
-        model.encoder.embeddings.copy_((torch.rand(model.encoder.embeddings.shape, generator=g) * 2 - 1) * 0.5)
-    return model.to(DEV).train()
-
-
-@pytest.mark.skipif(not STAGED, reason="reference files not staged")
-@pytest.mark.parametrize("bound", [1, 2], ids=["1cascade", "2cascades"])
-def test_full_update_matches_reference_python(bound, monkeypatch):
-    from nerf_texture_b200 import density
-    ntx()
-    ref_model = _random_model(bound)
-    our_model = copy.deepcopy(ref_model)
-    H3 = ref_model.grid_size ** 3
-    noise = torch.rand(ref_model.cascade, H3, 3, generator=torch.Generator().manual_seed(11)).to(DEV)
-    served = {"i": 0}
-
-    def fake_rand_like(t, *a, **k):                 # renderer.py:597 draws one [H^3, 3] block per cascade (S = 128: a single meshgrid block)
-        out = noise[served["i"] % ref_model.cascade]
-        served["i"] += 1
-        assert out.shape == t.shape
-        return out.clone()
-
-    for it in range(2):                             # two rounds: the second one exercises the decay of an already-populated grid
-        served["i"] = 0
-        monkeypatch.setattr(torch, "rand_like", fake_rand_like)
-        with torch.autocast("cuda", dtype=torch.half):
-            ref_model.update_extra_state()          # the reference's method, unmodified
-        monkeypatch.undo()
-        stats = density.update_density_grid(our_model.density_grid, our_model.density_bitfield, our_model.bound, our_model.density_scale,
-                                            our_model.density_thresh, our_model.encoder, our_model.sigma_net, decay=0.95, noise=noise)
-        torch.cuda.synchronize()
-        g_ref, g_our = ref_model.density_grid.cpu().numpy(), our_model.density_grid.cpu().numpy()
-        assert np.isfinite(g_our).all()
-        # same kernels' arithmetic on the same positions: the fused field kernel is bit-identical to grid encoder -> FFMLP (test_gpu_field.py)
-        np.testing.assert_array_equal(g_our, g_ref)
-        mean_ref = ref_model.mean_density
-        assert abs(float(stats[0]) - mean_ref) <= 1e-5 * max(1.0, abs(mean_ref))
-        thresh = min(mean_ref, ref_model.density_thresh)
-        b_ref, b_our = ref_model.density_bitfield.cpu().numpy(), our_model.density_bitfield.cpu().numpy()
-        diff = np.unpackbits(b_ref ^ b_our, bitorder="little").astype(bool)
-        # a bit may only differ where the density sits within rounding of the threshold (the two means differ in their last bits)
-        assert np.all(np.abs(g_ref.reshape(-1)[diff] - thresh) <= 1e-5 * max(1.0, thresh)), int(diff.sum())
 
 
 def test_density_update_vs_oracle_small_grid():

@@ -1,4 +1,5 @@
-"""GPU parity of the hash-grid encoder: libntx (through the C ABI) vs the CPU oracle and vs the reference's own CUDA.
+"""GPU parity of the hash-grid encoder: libntx (through the C ABI) vs the CPU oracle and vs the reference's own CUDA (its outputs
+on the same seeded inputs, stored in tests/golden/reference_outputs.npz).
 
 Bars (SURVEY.md F6 / section 8c):
   * integer corner-index streams: bit-exact vs the oracle (fed the device's per-level scales);
@@ -10,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from _util import cfgA, cfgB, cfgT, ntx, oracle, ref
+from _util import cfgA, cfgB, cfgT, ntx, oracle, ref, reference_output
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -112,9 +113,10 @@ def test_forward_pair_kernel_bit_exact(cfg, dtype):
     want = O.grid_encode(x, emb, offsets, pls, H, gridtype=0, align_corners=align, level_scales=scales)
     np.testing.assert_array_equal(got.view(np.uint16 if dtype == np.float16 else np.uint32),
                                   want.view(np.uint16 if dtype == np.float16 else np.uint32))
-    rgot, _ = _ref_forward(x, emb, offsets, pls, H, 0, align)
-    np.testing.assert_array_equal(got.view(np.uint16 if dtype == np.float16 else np.uint32),
-                                  rgot.view(np.uint16 if dtype == np.float16 else np.uint32))
+    bits = np.uint16 if dtype == np.float16 else np.uint32
+    rgot = reference_output("grid_pair_L%d_H%d_%s" % (kw["num_levels"], H, np.dtype(dtype).name),
+                            lambda: _ref_forward(x, emb, offsets, pls, H, 0, align)[0].view(bits), exact=True)
+    rgot.assert_equal(got.view(bits))
     # [L,B,C] layout of the same kernel
     got_lbc, _ = _ntx_forward(L_, x, emb, offsets, pls, H, 0, align, layout=0)
     nlev, C = kw["num_levels"], kw["level_dim"]
@@ -140,9 +142,15 @@ def test_forward_generic_and_dydx(D, C, gridtype, align, dtype):
     else:
         np.testing.assert_array_equal(got, want)
         np.testing.assert_array_equal(gdy, wdy)
-    rgot, rdy = _ref_forward(x, emb, offsets, pls, H, gridtype, align, calc=True)
-    np.testing.assert_array_equal(got, rgot)
-    np.testing.assert_array_equal(gdy, rdy)
+    key = "grid_generic_D%d_C%d_t%d_a%d_%s" % (D, C, gridtype, align, np.dtype(dtype).name)
+    live = {}
+
+    def ref_run(i):
+        if not live:
+            live["r"] = _ref_forward(x, emb, offsets, pls, H, gridtype, align, calc=True)
+        return live["r"][i]
+    reference_output(key + "_out", lambda: ref_run(0), exact=True).assert_equal(got)
+    reference_output(key + "_dydx", lambda: ref_run(1), exact=True).assert_equal(gdy)
 
 
 def test_out_of_range_rows_are_zero():
@@ -202,12 +210,14 @@ def test_backward_table_and_input_grads(cfg, dtype):
         assert err.max() <= 0.02 * scale + 1e-3, (err.max(), scale)
         assert np.abs(got_gi - gi64).max() <= 0.05 * np.abs(gi64).max()
     # the reference's own backward on the same inputs has the same kind of error; ours must not be worse by much
-    m = ref("gridencoder")
-    rge = torch.zeros_like(et)
-    rgi = torch.zeros(B, D, dtype=et.dtype, device=DEV)
-    glbc = gt.view(B, nlev, C).permute(1, 0, 2).contiguous()
-    m.grid_encode_backward(glbc, xt, et, ot, rge, B, D, C, nlev, float(np.log2(pls)), H, True, dyt, rgi, 0, align)
-    torch.cuda.synchronize()
-    ref_err = np.abs(rge.cpu().numpy().astype(np.float64) - ge64).max()
+    def ref_error():
+        m = ref("gridencoder")
+        rge = torch.zeros_like(et)
+        rgi = torch.zeros(B, D, dtype=et.dtype, device=DEV)
+        glbc = gt.view(B, nlev, C).permute(1, 0, 2).contiguous()
+        m.grid_encode_backward(glbc, xt, et, ot, rge, B, D, C, nlev, float(np.log2(pls)), H, True, dyt, rgi, 0, align)
+        torch.cuda.synchronize()
+        return np.abs(rge.cpu().numpy().astype(np.float64) - ge64).max()
+    ref_err = reference_output("grid_backward_L%d_%s_max_error" % (nlev, np.dtype(dtype).name), ref_error)
     our_err = np.abs(got_ge - ge64).max()
     assert our_err <= 2.0 * ref_err + 1e-6 * scale, (our_err, ref_err)

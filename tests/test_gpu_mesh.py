@@ -1,10 +1,6 @@
 """GPU parity tests of the mesh front end (SURVEY §8 f3) through the C ABI / the drop-in `RayTracer` and `frnn` packages:
-bit-exact against the oracle's exhaustive scans for the ray casts and the neighbour search, to tolerance for the fused projection
-(its reference is a chain of torch reductions), and the reference's UNMODIFIED MeshProjector.project on the drop-ins next to the fused
-kernel."""
-import os
-import sys
-
+bit-exact against the oracle's exhaustive scans for the ray casts and the neighbour search, and to tolerance for the fused projection
+(its reference is a chain of torch reductions)."""
 import numpy as np
 import pytest
 import torch
@@ -168,140 +164,10 @@ def test_project_against_oracle(sphere):
     assert (fi >= 0).float().mean() > 0.95
 
 
-def _reference_map():
-    sys.path.insert(0, os.path.join(U.ROOT, "tools"))
-    import run_reference_files as R
-    if not os.path.exists(os.path.join(R.STAGE, "callers", "tools", "map.py")):
-        pytest.skip("reference files not staged (tools/stage_reference.py)")
-    return R.import_reference_map()
-
-
-def _reference_projector(ref_map, v, f, vn):
-    """a MeshProjector of the reference's own class with the state its __init__ (trimesh / open3d / xatlas work) would leave behind"""
-    import frnn
-    from RayTracer import RayTracer
-    mp = ref_map.MeshProjector.__new__(ref_map.MeshProjector)
-    mp.mesh_vertices, mp.vertex_normals = _t(v), _t(vn)
-    _, _, _, mp.grid = frnn.frnn_grid_points(mp.mesh_vertices.unsqueeze(0), mp.mesh_vertices.unsqueeze(0), None, None, K=8, r=100., grid=None,
-                                             return_nn=False, return_sorted=True)                                  # map.py:396
-    mp.radius, mp.distance_method, mp.max_K = 100., "frnn", len(v)                                                 # map.py:397-399
-    mp.raytracer, mp.depth_threshold = RayTracer(v, f), 9.5                                                        # map.py:403,406
-    mp.faces = _t(f.astype(np.int64))
-    g = torch.Generator().manual_seed(0)
-    mp.tbn = torch.randn(len(f), 3, 3, generator=g).to(DEV)
-    mp.uvs = None
-    return mp
-
-
 def _shell_samples(n, seed):
     rng = np.random.default_rng(seed)
     x = rng.normal(size=(n, 3))
     return _t((x / np.linalg.norm(x, axis=1, keepdims=True) * rng.uniform(0.4, 1.0, (n, 1))).astype(np.float32))
-
-
-def test_unmodified_meshprojector_project_on_the_dropins(sphere):
-    """the reference's own tools/map.py, byte for byte: MeshProjector.project / .knn (map.py:414-500) run on the drop-in frnn and
-    RayTracer packages, and agree with the fused one-launch projection"""
-    ref_map = _reference_map()
-    from nerf_texture_b200 import mesh as M
-    v, f, vn, _ = sphere
-    mp = _reference_projector(ref_map, v, f, vn)
-    x = _shell_samples(30000, 11)
-    p_sur, sdf, h_mask, normal, tbn = mp.project(x, K=8, h_threshold=0.1)                                          # the reference's code
-    q_sur, qsdf, qmask, qnormal, qtbn = M.project(mp, x, K=8, h_threshold=0.1)                                     # one kernel
-    assert qsdf.shape == sdf.shape and qmask.shape == h_mask.shape and qtbn.shape == tbn.shape
-    _, _, d1, f1 = mp.raytracer.trace(x, normal)
-    _, _, d2, f2 = mp.raytracer.trace(x, -normal)
-    face_ref = torch.where(d1 < d2, f1, f2)                                                                        # map.py:425 (project() only returns tbn[face])
-    qface = mp._ntx_mesh.project(x, mp.vertex_normals, K=8)[3]
-    _project_tolerances((q_sur.cpu().numpy(), qsdf.cpu().numpy(), qnormal.cpu().numpy(), qface.cpu().numpy()),
-                        (p_sur.cpu().numpy(), sdf.cpu().numpy(), normal.cpu().numpy(), face_ref.cpu().numpy()), x.cpu().numpy(), "fused kernel vs reference chain")
-    agree = (qmask == h_mask).float().mean().item()
-    assert agree > 0.999
-    same = (qtbn == tbn).all(-1).all(-1).float().mean().item()
-    assert same > 0.998
-
-
-def test_unmodified_texture_field_runs_end_to_end(sphere):
-    """SURVEY 8 f3's purpose: the PRODUCT's field — the reference's unmodified MeshFeatureField (tools/map.py:546; cfgT hash grids, mesh
-    projection, factorised normal net) — constructs and evaluates on the drop-in packages alone (gridencoder, frnn, RayTracer), and gives
-    the same embedding with the projection swapped for the fused kernel"""
-    ref_map = _reference_map()
-    from nerf_texture_b200 import mesh as M
-    v, f, vn, _ = sphere
-    mp = _reference_projector(ref_map, v, f, vn)
-    original = ref_map.MeshProjector
-    ref_map.MeshProjector = lambda *a, **k: mp          # MeshFeatureField.__init__ builds its projector from a mesh FILE (trimesh): hand it ours
-    try:
-        torch.manual_seed(0)
-        field = ref_map.MeshFeatureField(mesh_path=None, h_threshold=0.1, K=8, bound=1).to(DEV)
-    finally:
-        ref_map.MeshProjector = original
-    with torch.no_grad():
-        field.encoder.embeddings.uniform_(-1, 1)        # the reference initialises to +-1e-4: make the features worth comparing
-    x = _shell_samples(20000, 21)
-    with torch.no_grad():
-        embed, n_coarse, n_fine, h_mask = field(x, no_noise=True)                                 # map.py:621: project -> encoders -> normal net
-    assert embed.shape == (20000, field.encoder_f_out_dim + field.encoder_z_outdim) and n_coarse.shape == (20000, 3) and n_fine.shape == (20000, 3)
-    assert h_mask.dtype == torch.bool and 0.1 < h_mask.float().mean().item() < 0.9
-    assert torch.isfinite(embed[h_mask]).all() and torch.isfinite(n_fine[h_mask]).all()
-    mp.project = lambda xyz, K=8, h_threshold=None, requires_grad_xyz=False, use_dir_vec=True: M.project(mp, xyz, K=K, h_threshold=h_threshold)
-    with torch.no_grad():
-        embed2, n_coarse2, n_fine2, h_mask2 = field(x, no_noise=True)
-    assert (h_mask == h_mask2).float().mean().item() > 0.999
-    both = h_mask & h_mask2
-    assert (n_coarse - n_coarse2).abs().max().item() < 1e-4
-    # p_sur moves by <= 1e-4 only where both projections landed on the same face; the hash-grid features are continuous in p_sur
-    close = ((embed - embed2).abs().max(dim=1)[0] < 2e-2) & ((n_fine - n_fine2).abs().max(dim=1)[0] < 2e-2)
-    assert close[both].float().mean().item() > 0.995
-
-
-def test_products_model_renders_through_the_unmodified_renderer(sphere):
-    """the PRODUCT end to end: the reference's unmodified nerf/network_curvedfield.py model (texture field on a mesh, tcnn networks) builds
-    its occupancy grid with the unmodified NeRFRenderer.update_extra_state and renders a frame through the unmodified
-    NeRFRenderer.render -> run_cuda, all on the drop-in packages (gridencoder, tinycudann, raymarching, frnn, RayTracer); swapping the
-    projection for the fused kernel gives the same picture"""
-    sys.path.insert(0, os.path.join(U.ROOT, "tools"))
-    import run_reference_files as R
-    if not os.path.exists(os.path.join(R.STAGE, "callers", "nerf", "network_curvedfield.py")):
-        pytest.skip("reference files not staged (tools/stage_reference.py)")
-    ref_map, NeRFNetwork = R.import_reference_product_model()
-    from nerf_texture_b200 import mesh as M
-    from nerf_texture_b200 import scene
-    v, f, vn, _ = sphere
-    mp = _reference_projector(ref_map, v, f, vn)
-    original = ref_map.MeshProjector
-    ref_map.MeshProjector = lambda *a, **k: mp
-    try:
-        torch.manual_seed(0)
-        model = NeRFNetwork(surface_mesh_path=None, light_model="None", bound=1, cuda_ray=True).to(DEV).eval()     # network_curvedfield.py:33
-    finally:
-        ref_map.MeshProjector = original
-    with torch.no_grad():
-        model.meshfea_field.encoder.embeddings.uniform_(-1, 1)
-    rays_o, rays_d = scene.pinhole_rays(96, 96, torch.device(DEV))
-
-    def frame():
-        with torch.no_grad(), torch.autocast("cuda", dtype=torch.half):
-            return model.render(rays_o[None], rays_d[None], staged=False, bg_color=1, perturb=False, max_steps=1024)
-
-    with torch.no_grad(), torch.autocast("cuda", dtype=torch.half):
-        model.update_extra_state()                                                              # renderer.py:567: density() of 128^3 cells -> bit-field
-    occupied = sum(bin(b).count("1") for b in model.density_bitfield.cpu().numpy().tobytes()) / (128.0 ** 3)
-    assert 0.01 < occupied < 0.6, occupied                                                      # the shell |sdf| < h_threshold around the mesh
-    out = frame()
-    image, depth = out["image"][0].float(), out["depth"][0].float()
-    assert image.shape == (96 * 96, 3) and torch.isfinite(image).all() and torch.isfinite(depth).all()
-    b = (rays_o * rays_d).sum(-1)
-    hits_ball = (b * b - ((rays_o * rays_o).sum(-1) - 0.55 ** 2)) > 0                           # rays through the inside of the bumpy sphere (r >= 0.6)
-    far_miss = (b * b - ((rays_o * rays_o).sum(-1) - 0.95 ** 2)) < 0                            # rays that pass outside the shell altogether
-    assert (image[far_miss] == 1).all() and (depth[far_miss] == 0).all()                        # background only
-    assert (image[hits_ball] < 0.999).any(dim=-1).float().mean() > 0.95                         # the shell absorbs something on every such ray
-    mp.project = lambda xyz, K=8, h_threshold=None, requires_grad_xyz=False, use_dir_vec=True: M.project(mp, xyz, K=K, h_threshold=h_threshold)
-    out2 = frame()
-    diff = (out2["image"][0].float() - image).abs()
-    # fp16 autocast + U(-1,1) features on a 1024-cell grid amplify the last-bit differences of the two projections (measured: 0.026 / 0.0026)
-    assert diff.max().item() < 0.1 and diff.mean().item() < 1e-2, (diff.max().item(), diff.mean().item())
 
 
 def test_morton_visit_order_changes_nothing(sphere):

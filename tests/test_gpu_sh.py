@@ -1,9 +1,10 @@
-"""GPU parity of the SH direction encoder vs the oracle (fp64 evaluation of the same polynomials) and the reference CUDA."""
+"""GPU parity of the SH direction encoder vs the oracle (fp64 evaluation of the same polynomials) and the reference CUDA (its outputs on
+the same inputs, stored in tests/golden/reference_outputs.npz)."""
 import numpy as np
 import pytest
 import torch
 
-from _util import ntx, oracle, ref
+from _util import ntx, oracle, ref, reference_output
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -40,15 +41,23 @@ def test_forward_and_dydx(degree, unit):
     tol = 8e-6 * max(1.0, np.abs(want).max())
     assert np.abs(got - want).max() <= tol
     assert np.abs(gdy - wdy).max() <= 2e-5 * max(1.0, np.abs(wdy).max())
-    m = ref("shencoder")
-    rout = torch.empty_like(out)
-    rdy = torch.empty_like(dy)
-    m.sh_encode_forward(dt, rout, B, 3, degree, True, rdy)
-    torch.cuda.synchronize()
-    rerr = np.abs(rout.cpu().numpy() - want).max()
-    assert np.abs(got - rout.cpu().numpy()).max() <= tol + rerr
+    live = {}
+
+    def ref_run(i):
+        if not live:
+            m = ref("shencoder")
+            rout = torch.empty_like(out)
+            rdy = torch.empty_like(dy)
+            m.sh_encode_forward(dt, rout, B, 3, degree, True, rdy)
+            torch.cuda.synchronize()
+            live["r"] = rout.cpu().numpy(), rdy.cpu().numpy()
+        return live["r"][i]
+    key = "sh_deg%d_%s" % (degree, "unit" if unit else "offsphere")
+    rerr = reference_output(key + "_max_error", lambda: np.abs(ref_run(0) - want).max())
+    rout, rdy = reference_output(key + "_out", lambda: ref_run(0)), reference_output(key + "_dydx", lambda: ref_run(1))
+    assert np.abs(rout.take(got) - rout.sample).max() <= tol + rerr
     assert np.abs(got - want).max() <= max(2 * rerr, tol)
-    assert np.abs(gdy - rdy.cpu().numpy()).max() <= 4e-5 * max(1.0, np.abs(wdy).max())
+    assert np.abs(rdy.take(gdy) - rdy.sample).max() <= 4e-5 * max(1.0, np.abs(wdy).max())
 
 
 def test_backward_accumulates():

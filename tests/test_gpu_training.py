@@ -1,10 +1,11 @@
 """GPU parity of the training path (BASELINE config 5): fused-MLP backward (activation + weight gradients), hash-grid table
-gradients through the drop-in modules' autograd, against fp64 references, the CPU oracle and the reference's own CUDA."""
+gradients through the drop-in modules' autograd, against fp64 references, the CPU oracle and the reference's own CUDA (its error on
+the same seeded inputs, stored in tests/golden/reference_outputs.npz)."""
 import numpy as np
 import pytest
 import torch
 
-from _util import ntx, oracle, ref, ulp16
+from _util import ntx, oracle, ref, reference_output, ulp16
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -70,17 +71,19 @@ def test_ffmlp_backward(din, hid, layers, B):
     gerr = np.abs(gi_n - tgin) / np.abs(tgin).max()
     assert np.median(gerr) < 1e-3 and np.mean(gerr > 3e-2) < 0.01, (np.median(gerr), np.mean(gerr > 3e-2))
     if B % 128 == 0 and hid >= 32:
-        m = ref("ffmlp")
-        m.allocate_splitk(layers + 1)
-        rout = torch.empty(B, 16, dtype=torch.half, device=DEV)
-        rfb = torch.empty(layers, B, hid, dtype=torch.half, device=DEV)
-        m.ffmlp_forward(xt, wt, B, din, 16, hid, layers, 0, 6, rfb, rout)
-        rbb = torch.zeros(layers, B, hid, dtype=torch.half, device=DEV)
-        rgi = torch.zeros(B, din, dtype=torch.half, device=DEV)
-        rgw = torch.zeros_like(wt)
-        m.ffmlp_backward(gt, xt, wt, rfb, B, din, 16, hid, layers, 0, 6, True, rbb, rgi, rgw)
-        torch.cuda.synchronize()
-        err_ref = np.abs(rgw.cpu().numpy().astype(np.float64) - tgw).max() / np.abs(tgw).max()
+        def ref_error():
+            m = ref("ffmlp")
+            m.allocate_splitk(layers + 1)
+            rout = torch.empty(B, 16, dtype=torch.half, device=DEV)
+            rfb = torch.empty(layers, B, hid, dtype=torch.half, device=DEV)
+            m.ffmlp_forward(xt, wt, B, din, 16, hid, layers, 0, 6, rfb, rout)
+            rbb = torch.zeros(layers, B, hid, dtype=torch.half, device=DEV)
+            rgi = torch.zeros(B, din, dtype=torch.half, device=DEV)
+            rgw = torch.zeros_like(wt)
+            m.ffmlp_backward(gt, xt, wt, rfb, B, din, 16, hid, layers, 0, 6, True, rbb, rgi, rgw)
+            torch.cuda.synchronize()
+            return np.abs(rgw.cpu().numpy().astype(np.float64) - tgw).max() / np.abs(tgw).max()
+        err_ref = reference_output("ffmlp_backward_%d_%d_%d_%d_weight_grad_error" % (din, hid, layers, B), ref_error)
         assert err_ours <= err_ref * 1.1 + 1e-3, (err_ours, err_ref)     # fp32 accumulation must not be worse than the reference's fp16 split-K
 
 

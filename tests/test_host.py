@@ -44,6 +44,7 @@ def test_grid_encoder_state_matches_reference_layout():
     t = GridEncoder(num_levels=4, log2_hashmap_size=14, gridtype="tiled")
     assert t.gridtype_id == 1 and np.diff(t.offsets.numpy()).tolist() == [4920, 16384, 16384, 16384]
     c = GridEncoder_clustering(num_levels=4, log2_hashmap_size=12)
+    c = c.to(c.cluster_layers[0].cluster_centers.device)                  # the centres start on the GPU when there is one, like the reference's
     assert len(c.cluster_layers) == 4 and float(c.clustering_loss(pick_level=False)) == pytest.approx(float(c.clustering_loss(pick_level=False)))
 
 
