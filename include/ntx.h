@@ -283,6 +283,30 @@ int ntx_mesh_knn(const void* mesh, const float* queries, uint32_t N, uint32_t K,
 int ntx_mesh_project(const void* mesh, const float* vertex_normals, const float* xyz, uint32_t N, uint32_t K, float r, float dir_vec_wdist,
                      float* p_sur, float* sdf, float* normal, int64_t* face_idx, ntx_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------------------------------------------
+ * Fused texture-field density: NeRFNetwork.density(x) of the product's model (nerf/network_curvedfield.py:412-433) in fp16 inference,
+ * for the configuration main.py trains (MeshFeatureField with hash=True, prob_model=False, no imported texture; sigma_net = tcnn
+ * FullyFusedMLP, ReLU, one hidden layer of 32 neurons, no output activation), as ONE kernel:
+ *   MeshProjector.project(xyz, K) as in ntx_mesh_project (tools/map.py:414-433) -> p_sur, sdf
+ *   x_embed = texture grid at (p_sur + bound) / (2 bound)  (tools/map.py:563,623; D = 3, C = 2, L levels, every level hashed, fp16 table
+ *             as under autocast; out-of-range coordinates — casts that miss may leave the box — give zero features, like the reference)
+ *   z_embed = FreqEncoder(sdf) = [sdf, sin(2^i sdf), cos(2^i sdf) for i = 0..11]  (tools/encoding.py:5-43, get_encoder('frequency', multires=12))
+ *   h = sigma_net(cat(x_embed, z_embed) zero-padded to 16*ceil((2L+25)/16), rounded to fp16)  (tools/map.py:719, network_curvedfield.py:416)
+ *   sigma = |sdf| < h_threshold ? exp(float(h[0])) : 0        (trunc_exp + torch.where, network_curvedfield.py:417-421)
+ *   h_threshold = min(MeshProjector.depth_threshold, MeshFeatureField.h_threshold) as fp32 (tools/map.py:429-431)
+ *   mesh, vertex_normals, K, r, dir_vec_wdist as in ntx_mesh_project; embeddings_f16, offsets, L, S, H, align_corners as in
+ *   ntx_ngp_field_forward.  w_sigma_f16: the tinycudann shim's flat parameters [32 x in | 16 x 32] fp16, each matrix row-major [out,in].
+ *   xyz [N,3] f32 -> sigma [N] f32, h_f16 [N,16] fp16 (geo_feat = h[:, 1:]).  w_sigma_f16 and h_f16 16-byte aligned.
+ * Every sample gets h, also those outside the shell (sigma 0) and those whose casts miss (sdf = 10).  A null or triangle-less mesh,
+ * K outside 1..16 or L outside 1..32 -> NTX_ERR_INVALID_ARGUMENT (checked before the device is touched, except the triangle count);
+ * N = 0 is a no-op.  Queries are independent: like ntx_mesh_project, a batch in Morton order runs faster.
+ * Measured on one B200 (1000 W power limit), 2^20 samples around a 230 K-triangle mesh: 5.54 ms, against 4.74 ms for the same computation
+ * composed from the drop-in operators — not yet faster, see DESIGN.md §4.10 (profiles/r03_texture_field.txt). */
+int ntx_texture_field_density(const void* mesh, const float* vertex_normals, const float* xyz, uint32_t N, uint32_t K, float r,
+                              float dir_vec_wdist, float h_threshold, float bound, const void* embeddings_f16, const int* offsets,
+                              uint32_t L, float S, uint32_t H, int align_corners, const void* w_sigma_f16, float* sigma, void* h_f16,
+                              ntx_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

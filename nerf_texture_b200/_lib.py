@@ -52,6 +52,7 @@ _SIGS = {
     "ntx_mesh_trace": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _u32, _vp],
     "ntx_mesh_knn": [_vp, _vp, _u32, _u32, _f32, _vp, _vp, _vp],
     "ntx_mesh_project": [_vp, _vp, _vp, _u32, _u32, _f32, _f32, _vp, _vp, _vp, _vp, _vp],
+    "ntx_texture_field_density": [_vp, _vp, _vp, _u32, _u32, _f32, _f32, _f32, _f32, _vp, _vp, _u32, _f32, _u32, _int, _vp, _vp, _vp, _vp],
     "ntx_update_density_grid": [_vp, _vp, _u32, _u32, _f32, _f32, _f32, _f32, _vp, _vp, _u32, _f32, _u32, _int, _vp, _vp, _u32, _vp, _int, _vp, _vp, _vp],
 }
 _SIZE_FNS = {

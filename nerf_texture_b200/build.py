@@ -19,7 +19,8 @@ LIBDIR = os.path.join(HERE, "lib")
 _TAG = os.environ.get("NTX_BUILD_TAG", "")
 OBJDIR = os.path.join(LIBDIR, "obj" + ("_" + _TAG if _TAG else ""))
 LIB = os.path.join(LIBDIR, "libntx" + ("_" + _TAG if _TAG else "") + ".so")
-SOURCES = ["api.cu", "grid.cu", "sh.cu", "raymarch.cu", "mlp.cu", "mlp_bwd.cu", "field.cu", "mesh.cu"]
+# longest compile first (mlp.cu: ~55 s of ~100 s in all), so that a build with fewer jobs than sources is not left waiting on it at the end
+SOURCES = ["mlp.cu", "grid.cu", "mlp_bwd.cu", "mesh.cu", "texture_field.cu", "raymarch.cu", "field.cu", "sh.cu", "api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--expt-relaxed-constexpr", "-Xptxas", "-v",
@@ -64,10 +65,42 @@ def _compile(src, force, verbose):
     return obj, True, r.stderr
 
 
+def _mem_available_bytes():
+    """memory this process can still use: MemAvailable, or less under a cgroup (v2) memory limit; None if unknown"""
+    avail = None
+    try:
+        with open("/proc/meminfo") as f:
+            avail = next(int(l.split()[1]) * 1024 for l in f if l.startswith("MemAvailable:"))
+    except (OSError, StopIteration, ValueError):
+        pass
+    try:
+        with open("/sys/fs/cgroup/memory.max") as f:
+            limit = f.read().strip()
+        if limit != "max":
+            with open("/sys/fs/cgroup/memory.current") as f:
+                free = int(limit) - int(f.read().strip())
+            avail = free if avail is None else min(avail, free)
+    except (OSError, ValueError):
+        pass
+    return avail
+
+
+def _jobs(n):
+    """parallel nvcc jobs: no more than the CPUs this process may run on (os.cpu_count() counts the host's in a container) and one per
+    GB of available memory (cicc + ptxas of mlp.cu peak at ~0.6 GB, the other sources at ~0.25 GB)"""
+    try:
+        cpus = len(os.sched_getaffinity(0))
+    except (AttributeError, OSError):
+        cpus = os.cpu_count() or 4
+    mem = _mem_available_bytes()
+    by_mem = max(1, mem // (1 << 30)) if mem is not None else cpus
+    return max(1, min(n, cpus, by_mem))
+
+
 def build(force=False, verbose=False):
     os.makedirs(OBJDIR, exist_ok=True)
     srcs = [s for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
-    with ThreadPoolExecutor(max_workers=min(len(srcs), os.cpu_count() or 4)) as ex:
+    with ThreadPoolExecutor(max_workers=_jobs(len(srcs))) as ex:
         results = list(ex.map(lambda s: _compile(s, force, verbose), srcs))
     objs = [r[0] for r in results]
     rebuilt = any(r[1] for r in results)

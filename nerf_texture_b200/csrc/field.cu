@@ -40,7 +40,6 @@ constexpr int kTasksPerTile = 8;                                         // kTil
 constexpr int kFieldThreads = 32 * (kConsumerWarps + kProducerWarps);   // 512
 constexpr int kFW = 64;          // hidden width of both MLPs
 constexpr int kColorIn = 32;     // SH(16) + geo_feat(15) + zero pad (network_ff.py:42,95-97)
-constexpr int kFieldMaxLevels = 32;
 constexpr int kStages = NTX_FIELD_STAGES;       // feature tiles in the producer -> consumer ring
 #ifndef NTX_FIELD_CTX
 #define NTX_FIELD_CTX 1
@@ -110,44 +109,15 @@ __device__ __forceinline__ void field_hidden_epilogue(uint32_t acc, uint32_t opn
 //   st = ns+1       h [128 x 32] . Wc0^T  -> 64      hidden epilogue
 //   st = ns+2..ns+nc                      -> 64      hidden epilogue
 //   st = ns+nc+1    h . Wc_out^T          -> 16      rgb
-// Everything the issuing lane needs for the MMAs of stage st (1 .. ns+nc+1), precomputed once per CTA: between the consumers' barrier
-// and the first UTCHMMA of a stage the round-2 build spent ~50 uniform-datapath instructions assembling descriptors (SASS) — on the
-// critical path of every stage, issued by one warp while the other three wait, next to twelve gathering warps.
-struct StageMma {
-    uint32_t b_lo[4];      // low words of the weight (B operand) descriptors of the K = 16 steps
-    uint32_t b_hi;         // their common high word (SBO, descriptor version)
-    uint32_t idesc;        // instruction descriptor (M = 128, N = 64 or 16)
-    uint32_t ksteps;       // 2 (the colour net's 32-wide input) or 4
-    uint32_t pad;
-};
-static_assert(sizeof(StageMma) == 32, "StageMma is two 16-byte loads");
+// The MMAs of stage st come from a StageMma table (mlp_tile.cuh) precomputed once per CTA: between the consumers' barrier and the
+// first UTCHMMA of a stage the round-2 build spent ~50 uniform-datapath instructions assembling descriptors (SASS) — on the critical
+// path of every stage, issued by one warp while the other three wait, next to twelve gathering warps.
 __device__ __forceinline__ StageMma make_stage_mma(uint32_t st, uint32_t ns, uint32_t nc, uint32_t K0, uint32_t ws_addr, uint32_t wc_addr) {
     uint32_t w, Kdim, N;
     if (st <= ns) { w = ws_addr + kFW * K0 * 2u + (st - 1) * (kFW * kFW * 2u); Kdim = kFW; N = st == ns ? 16u : (uint32_t)kFW; }
     else if (st == ns + 1) { w = wc_addr; Kdim = kColorIn; N = kFW; }
     else { w = wc_addr + kFW * kColorIn * 2u + (st - ns - 2) * (kFW * kFW * 2u); Kdim = kFW; N = st == ns + nc + 1 ? 16u : (uint32_t)kFW; }
-    StageMma m;
-    m.ksteps = Kdim >> 4;
-    m.idesc = tc::idesc_f16_f32(kTileRows, N);
-    m.b_hi = 0; m.pad = 0;
-    for (uint32_t ks = 0; ks < 4; ks++) {
-        const uint64_t d = tc::smem_desc_kmajor_noswz(w + (ks < m.ksteps ? ks : 0u) * 256u, 128u, Kdim * 16u);
-        m.b_lo[ks] = (uint32_t)d;
-        m.b_hi = (uint32_t)(d >> 32);
-    }
-    return m;
-}
-// issue stage st from its table entry: A = the operand columns in tensor memory (8 per K = 16 step)
-__device__ __forceinline__ void field_issue_stage(const StageMma* __restrict__ table, uint32_t st, uint32_t tmem_a, uint32_t tmem_acc) {
-    const uint4 lo = *reinterpret_cast<const uint4*>(table[st].b_lo);
-    const uint4 meta = *reinterpret_cast<const uint4*>(&table[st].b_hi);        // b_hi, idesc, ksteps, pad
-    const uint64_t hi = (uint64_t)meta.x << 32;
-    tc::mma_f16_ts(tmem_acc, tmem_a, hi | lo.x, meta.y, 0u);
-    tc::mma_f16_ts(tmem_acc, tmem_a + 8u, hi | lo.y, meta.y, 1u);
-    if (meta.z == 4u) {
-        tc::mma_f16_ts(tmem_acc, tmem_a + 16u, hi | lo.z, meta.y, 1u);
-        tc::mma_f16_ts(tmem_acc, tmem_a + 24u, hi | lo.w, meta.y, 1u);
-    }
+    return stage_mma(w, Kdim, N);
 }
 
 // What a row is: MODE_ROWS  = a row of xyz/dirs (the ntx_ngp_field_forward contract, optionally through a row list);
@@ -429,7 +399,7 @@ __global__ void __launch_bounds__(kFieldThreads, 2) ngp_field_kernel(
                     tc::tmem_wait_st(); tc::tc_fence_before_sync(); consumer_sync();
                     if (st + 1 < nst && warp == 0 && tc::elect_one()) {
                         tc::tc_fence_after_sync();
-                        field_issue_stage(stage_table, st + 1, opnd_all, acc_all);
+                        issue_stage_ts(stage_table, st + 1, opnd_all, acc_all);
                         tc::mma_commit(&mma_bar[c]);
                     }
                     PROBE_MARK(2)

@@ -6,6 +6,8 @@
 
 namespace ntx {
 
+constexpr int kFieldMaxLevels = 32;      // levels the fused kernels (field.cu, texture_field.cu) keep in their shared level table
+
 // ---------------------------------------------------------------------------------------------------- level table
 struct GridLevel {
     float scale;         // exp2f(level*S)*H - 1                      gridencoder.cu:126

@@ -8,29 +8,14 @@
 // stack in local memory, the K-entry neighbour list in registers) is small.  Two other mappings were built, verified bit-exact and
 // measured slower on B200 (DESIGN.md, "Tried and lost"; profiles/r02_mesh_ab_*): lanes pulling queries from a per-warp chunk, and
 // 8 lanes per query on an 8-wide tree.
-#include "common.cuh"
 #include "mesh_build.h"
+#include "mesh_project.cuh"
 
 #include <mutex>
 #include <new>
 
 namespace ntx {
 namespace mesh {
-
-constexpr uint32_t kMeshMagic = 0x4d53484eu;
-
-struct MeshHandle {
-    uint32_t magic;
-    int device;
-    uint32_t n_vertices, n_triangles;
-    uint32_t tri_nodes_n, pt_nodes_n, tri_depth, pt_depth;
-    float slack;          // pruning slack of trace_one: 1e-5 of the mesh's largest extent
-    Node* tri_nodes;
-    Tri* tris;
-    Node* pt_nodes;
-    Point* pts;
-    float* vertices;      // [n_vertices, 3] in the caller's order (the fused projection gathers neighbours by index)
-};
 
 static void free_handle(MeshHandle* h) {
     if (!h) return;
@@ -46,10 +31,6 @@ static bool upload(T** dst, const std::vector<T>& src) {
     if (cudaMalloc((void**)dst, bytes) != cudaSuccess) return false;
     if (!src.empty() && cudaMemcpy(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) return false;
     return true;
-}
-
-__device__ __forceinline__ void load3(const float* p, uint32_t i, float* v) {
-    v[0] = p[3 * (size_t)i]; v[1] = p[3 * (size_t)i + 1]; v[2] = p[3 * (size_t)i + 2];
 }
 
 // bvh.cu:695-721 raytrace_kernel.  positions may alias rays_o and normals rays_d (raytracer.py:52-54 `inplace`): a thread reads its
@@ -96,96 +77,21 @@ __global__ void __launch_bounds__(128) mesh_knn_kernel(uint32_t N, const float* 
     }
 }
 
-__device__ __forceinline__ float norm3(const float* v) { return sqrtf(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]); }
-
-// tools/map.py:454-500 (knn with use_dir_vec=True, weighting='Shepard'): the terms one neighbour contributes.  The arithmetic is plain
-// fp32 (the reference's is a chain of ~30 torch kernels over [N,K,3] temporaries whose reduction order is not specified — parity is to
-// tolerance there, see the tests).  sums = {mean_dir[3], normal_test[3], weighted normals[3], weight sum}
-__device__ __forceinline__ void neighbour_terms(const float* x, bool ok, float d2, int idx, const float* __restrict__ vertices,
-                                                const float* __restrict__ vertex_normals, uint32_t n_vertices, float* sums) {
-    // fewer than K vertices in the radius: frnn pads with -1, which torch's indexing wraps to the last vertex, sqrt(-1) = NaN (:458)
-    const uint32_t j = ok ? (uint32_t)idx : n_vertices - 1;
-    const float dis = ok ? sqrtf(d2) : NAN;
-    float vn[3], dvo[3];
-    for (int c = 0; c < 3; c++) { vn[c] = __ldg(vertex_normals + 3 * (size_t)j + c); dvo[c] = x[c] - __ldg(vertices + 3 * (size_t)j + c); }
-    const float len = norm3(dvo) + 1e-5f;                 // :461
-    const float w = 1.0f / (dis + 1e-7f);                 // :474 and :487 (Shepard): the same weight twice
-    const float nl = norm3(vn) + 1e-5f;                   // :497
-    for (int c = 0; c < 3; c++) {
-        sums[c] += w * (dvo[c] / len);                    // :476
-        sums[3 + c] += vn[c];                             // :477
-        sums[6 + c] += (vn[c] / nl) * w;                  // :498 before the division by the weight sum
-    }
-    sums[9] += w;
-}
-
-__device__ __forceinline__ void finish_normal(float* sums, int k_want, float dir_vec_wdist, float* n) {
-    float* mean_dir = sums;
-    float* ntest = sums + 3;
-    float* acc = sums + 6;
-    float wsum = sums[9];
-    for (int c = 0; c < 3; c++) ntest[c] /= (float)k_want;
-    if (mean_dir[0] * ntest[0] + mean_dir[1] * ntest[1] + mean_dir[2] * ntest[2] < 0.0f)
-        for (int c = 0; c < 3; c++) mean_dir[c] = -mean_dir[c];  // :478
-    {
-        const float len = norm3(mean_dir) + 1e-5f;                // :479
-        for (int c = 0; c < 3; c++) mean_dir[c] /= len;
-        const float w = 1.0f / (fmaxf(dir_vec_wdist, 1e-5f) + 1e-7f);   // :481-482, :487
-        const float nl = norm3(mean_dir) + 1e-5f;                 // :497 (normalised a second time, as the reference does)
-        for (int c = 0; c < 3; c++) acc[c] += (mean_dir[c] / nl) * w;
-        wsum += w;
-    }
-    for (int c = 0; c < 3; c++) acc[c] /= wsum;                   // :496
-    const float len = norm3(acc) + 1e-5f;                         // :499
-    for (int c = 0; c < 3; c++) n[c] = acc[c] / len;
-}
-
-// tools/map.py:421-425 after the two casts of :419-420
-__device__ __forceinline__ void project_outputs(size_t i, const float* x, const float* n, const Hit& h1, const Hit& h2, float* p_sur, float* sdf,
-                                                float* normal_out, long long* face_idx) {
-    const bool cond = h1.t < h2.t;                                 // :421
-    const float t = cond ? h1.t : h2.t;
-    for (int c = 0; c < 3; c++) {
-        p_sur[3 * i + c] = NTX_ADD(x[c], NTX_MUL(t, cond ? n[c] : -n[c]));   // :422
-        normal_out[3 * i + c] = n[c];
-    }
-    sdf[i] = cond ? -h1.t : h2.t;                                  // :423
-    face_idx[i] = cond ? h1.face : h2.face;                        // :425
-}
-
-// MeshProjector.project, one thread per sample: the neighbour list never leaves the registers, both casts run back to back
+// MeshProjector.project, one thread per sample (project_query)
 template <int K>
-__global__ void __launch_bounds__(128) mesh_project_kernel(uint32_t N, const float* xyz, int k_want, float r2, float dir_vec_wdist,
-                                                           const float* __restrict__ vertices, const float* __restrict__ vertex_normals,
-                                                           uint32_t n_vertices, const Node* __restrict__ pt_nodes, const Point* __restrict__ pts,
-                                                           const Node* __restrict__ tri_nodes, const Tri* __restrict__ tris, float slack,
+__global__ void __launch_bounds__(128) mesh_project_kernel(uint32_t N, const float* xyz, int k_want, float r2, float dir_vec_wdist, const MeshView m,
                                                            float* p_sur, float* sdf, float* normal_out, long long* face_idx) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
     float x[3];
     load3(xyz, i, x);
-    float bd[K];
-    int bi[K];
-    knn_one<K>(pt_nodes, pts, x, r2, k_want, bd, bi);
-    float sums[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-#pragma unroll
-    for (int s = 0; s < K; s++)
-        if (s >= K - k_want) neighbour_terms(x, knn_slot_valid(bi[s]), bd[s], bi[s], vertices, vertex_normals, n_vertices, sums);
-    float n[3], nn[3];
-    finish_normal(sums, k_want, dir_vec_wdist, n);
-    for (int c = 0; c < 3; c++) nn[c] = -n[c];
-    const Hit h1 = trace_one(tri_nodes, tris, x, n, slack);        // :419 inner
-    const Hit h2 = trace_one(tri_nodes, tris, x, nn, slack);       // :420 outer
-    project_outputs(i, x, n, h1, h2, p_sur, sdf, normal_out, face_idx);
-}
-
-static MeshHandle* checked(const void* mesh, const char* who) {
-    MeshHandle* h = (MeshHandle*)mesh;
-    if (!h || h->magic != kMeshMagic) { set_error("%s: not a mesh handle", who); return nullptr; }
-    int dev = -1;
-    cudaGetDevice(&dev);
-    if (dev != h->device) { set_error("%s: the mesh lives on device %d, the current device is %d", who, h->device, dev); return nullptr; }
-    return h;
+    const Projection p = project_query<K>(x, k_want, r2, dir_vec_wdist, m);
+    for (int c = 0; c < 3; c++) {
+        p_sur[3 * (size_t)i + c] = p.p_sur[c];
+        normal_out[3 * (size_t)i + c] = p.normal[c];
+    }
+    sdf[i] = p.sdf;
+    face_idx[i] = p.face;
 }
 
 }  // namespace mesh
@@ -298,12 +204,11 @@ int ntx_mesh_project(const void* mesh, const float* vertex_normals, const float*
     const float r2 = r * r;
     const uint32_t block = (uint32_t)tunables().mesh_block;
     const dim3 grid(ceil_div(N, block));
+    const MeshView m = mesh_view(h, vertex_normals);
     if (K <= 8) {
-        mesh_project_kernel<8><<<grid, block, 0, st>>>(N, xyz, (int)K, r2, dir_vec_wdist, h->vertices, vertex_normals, h->n_vertices, h->pt_nodes, h->pts,
-                                                     h->tri_nodes, h->tris, h->slack, p_sur, sdf, normal, (long long*)face_idx);
+        mesh_project_kernel<8><<<grid, block, 0, st>>>(N, xyz, (int)K, r2, dir_vec_wdist, m, p_sur, sdf, normal, (long long*)face_idx);
     } else {
-        mesh_project_kernel<16><<<grid, block, 0, st>>>(N, xyz, (int)K, r2, dir_vec_wdist, h->vertices, vertex_normals, h->n_vertices, h->pt_nodes, h->pts,
-                                                      h->tri_nodes, h->tris, h->slack, p_sur, sdf, normal, (long long*)face_idx);
+        mesh_project_kernel<16><<<grid, block, 0, st>>>(N, xyz, (int)K, r2, dir_vec_wdist, m, p_sur, sdf, normal, (long long*)face_idx);
     }
     return check_launch("ntx_mesh_project");
 }

@@ -57,6 +57,42 @@ __device__ __forceinline__ void issue_layer(uint32_t a_smem, uint32_t w_smem, ui
     }
 }
 
+// Everything the issuing lane needs for the MMAs of one layer whose A operand is in tensor memory, precomputed once per CTA
+// (field.cu, texture_field.cu): the layer is two LDS.128 + the UTCHMMAs instead of a descriptor build on the consumers' critical path.
+struct StageMma {
+    uint32_t b_lo[4];      // low words of the weight (B operand) descriptors of the K = 16 steps
+    uint32_t b_hi;         // their common high word (SBO, descriptor version)
+    uint32_t idesc;        // instruction descriptor (M = 128, N)
+    uint32_t ksteps;       // 2 (a 32-wide input) or 4 (64-wide)
+    uint32_t pad;
+};
+static_assert(sizeof(StageMma) == 32, "StageMma is two 16-byte loads");
+// weights W [N x Kdim] K-major at shared address w, Kdim = 32 or 64
+__device__ __forceinline__ StageMma stage_mma(uint32_t w, uint32_t Kdim, uint32_t N) {
+    StageMma m;
+    m.ksteps = Kdim >> 4;
+    m.idesc = tc::idesc_f16_f32(kTileRows, N);
+    m.b_hi = 0; m.pad = 0;
+    for (uint32_t ks = 0; ks < 4; ks++) {
+        const uint64_t d = tc::smem_desc_kmajor_noswz(w + (ks < m.ksteps ? ks : 0u) * 256u, 128u, Kdim * 16u);
+        m.b_lo[ks] = (uint32_t)d;
+        m.b_hi = (uint32_t)(d >> 32);
+    }
+    return m;
+}
+// issue layer st from its table entry: A = the operand columns in tensor memory (8 per K = 16 step)
+__device__ __forceinline__ void issue_stage_ts(const StageMma* __restrict__ table, uint32_t st, uint32_t tmem_a, uint32_t tmem_acc) {
+    const uint4 lo = *reinterpret_cast<const uint4*>(table[st].b_lo);
+    const uint4 meta = *reinterpret_cast<const uint4*>(&table[st].b_hi);        // b_hi, idesc, ksteps, pad
+    const uint64_t hi = (uint64_t)meta.x << 32;
+    tc::mma_f16_ts(tmem_acc, tmem_a, hi | lo.x, meta.y, 0u);
+    tc::mma_f16_ts(tmem_acc, tmem_a + 8u, hi | lo.y, meta.y, 1u);
+    if (meta.z == 4u) {
+        tc::mma_f16_ts(tmem_acc, tmem_a + 16u, hi | lo.z, meta.y, 1u);
+        tc::mma_f16_ts(tmem_acc, tmem_a + 24u, hi | lo.w, meta.y, 1u);
+    }
+}
+
 // activation ids of the reference (ffmlp.cu:22-33); applied to the fp16-rounded pre-activation like utils.h:425-470
 __device__ __forceinline__ float mlp_activation(uint32_t act, float x) {
     constexpr float K_ACT = 10.0f;

@@ -142,14 +142,20 @@ class Mesh:
         return p_sur.view(*prefix, 3), sdf.view(*prefix, 1), normal.view(*prefix, 3), face_idx.view(*prefix)
 
 
-def project(projector, xyz, K=8, h_threshold=None):
-    """Drop-in body for `MeshProjector.project(xyz, K, h_threshold)` (tools/map.py:414): `projector` is the reference's object (it needs
-    `.mesh_vertices`, `.vertex_normals`, `.tbn`, `.depth_threshold`, `.radius` and a mesh with faces); the handle is cached on it.
-    Returns p_sur, sdf, h_mask, normal, tbn like the reference."""
+def projector_mesh(projector):
+    """The Mesh of the reference's `MeshProjector` (`.mesh_vertices` and `.faces` or `.mesh.faces`), built on first use and cached on it."""
     m = getattr(projector, "_ntx_mesh", None)
     if m is None:
         faces = projector.faces if getattr(projector, "faces", None) is not None else projector.mesh.faces
         m = projector._ntx_mesh = Mesh(projector.mesh_vertices, faces, device=projector.mesh_vertices.device)
+    return m
+
+
+def project(projector, xyz, K=8, h_threshold=None):
+    """Drop-in body for `MeshProjector.project(xyz, K, h_threshold)` (tools/map.py:414): `projector` is the reference's object (it needs
+    `.mesh_vertices`, `.vertex_normals`, `.tbn`, `.depth_threshold`, `.radius` and a mesh with faces); the handle is cached on it.
+    Returns p_sur, sdf, h_mask, normal, tbn like the reference."""
+    m = projector_mesh(projector)
     p_sur, sdf, normal, face_idx = m.project(xyz, projector.vertex_normals, K=min(K, m.n_vertices), r=projector.radius)
     tbn = projector.tbn[face_idx] if getattr(projector, "tbn", None) is not None else None
     thr = projector.depth_threshold if h_threshold is None else min(projector.depth_threshold, h_threshold)
